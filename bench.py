@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- AlexNet product-quantized forward throughput (images/s) on N B200s, the metric of BASELINE.json.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -15,6 +15,8 @@ batch-sharded, weights replicated, and for N > 1 the only exchange is one all-ga
             measured peaks of MEASURED_PEAKS.json
   cpu_baseline  the reference's own CPU path timed on this box (rank 0, N = 1 only, bounded sample)
 `--impl reference` times the reference CPU implementation with all host cores instead (no GPU work at all).
+`--dump-outputs DIR` writes what the last timed step returned to its caller (rank 0: probabilities and logits) as
+DIR/prob.npy and DIR/logits.npy, float32; the inputs depend only on the arguments, so two builds can be compared.
 """
 import argparse
 import importlib
@@ -117,6 +119,22 @@ def model_files(writer, tmpdir):
         return REAL_DIR, REAL_PFX, "shipped quantized AlexNet (bvlc_alexnet_aCaF)"
     write_synthetic_alexnet(writer, tmpdir, "synth")
     return tmpdir, "synth", "random-init AlexNet PQ architecture"
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(dirpath, arrays):
+    """Writes every array as dirpath/<name>.npy in float32.  Above DUMP_LIMIT bytes in all, each keeps the same fixed,
+    seeded sample of its rows, so that dumps of two runs with the same arguments line up row for row."""
+    os.makedirs(dirpath, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT:
+            keep = max(1, a.shape[0] * DUMP_LIMIT // total)
+            a = a[np.sort(np.random.RandomState(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(dirpath, name + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -388,6 +406,10 @@ def run_b200_arm(args, q):
     barrier()
     if in_range:
         torch.cuda.cudart().cudaProfilerStop()
+    if args.dump_outputs and rank == 0:
+        # what the last step's caller received: this rank's probabilities and the logits (gathered over all ranks)
+        last_logits = gather.full[(args.steps - 1) & 1] if world > 1 else logits
+        dump_outputs(args.dump_outputs, {"prob": prob.cpu().numpy(), "logits": last_logits.cpu().numpy()})
     ms_total = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(ms_total, op=dist.ReduceOp.MAX)
@@ -736,7 +758,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-config4", action="store_true", help="skip the 1024-per-GPU (configs[3]) timing")
     ap.add_argument("--no-strict", action="store_true", help="skip the strict-path (tensor_core = 0) timing")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if args.impl == "reference":
         return run_reference_arm(args)
     q = importlib.import_module("quantized-cnn_b200")   # raises if libqcnn_b200.so is missing: no fallback

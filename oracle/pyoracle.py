@@ -370,6 +370,52 @@ def save_model(dirpath, pfx, params):
 
 
 # ------------------------------------------------------------------------------------------------
+# seeded stand-in for the reference's data directory
+# ------------------------------------------------------------------------------------------------
+SYNTH_BMP_SHAPES = [(375, 500), (333, 500), (500, 375), (256, 256), (227, 301), (480, 640), (301, 227), (257, 383),
+                    (400, 299), (281, 421)]      # (H, W): several row paddings, up- and down-scaling
+
+
+def write_bmp(path, pix):
+    """uint8 [H, W, 3] (B, G, R, top row first) -> 24-bpp uncompressed bottom-up BMP."""
+    h, w, _ = pix.shape
+    row = (w * 3 + 3) & ~3
+    body = np.zeros((h, row), np.uint8)
+    body[:, :w * 3] = pix[::-1].reshape(h, w * 3)
+    head = np.zeros(54, np.uint8)
+    head[0:2] = [ord("B"), ord("M")]
+    head[2:6] = np.frombuffer(np.uint32(54 + body.size).tobytes(), np.uint8)
+    head[10:14] = np.frombuffer(np.uint32(54).tobytes(), np.uint8)
+    head[14:18] = np.frombuffer(np.uint32(40).tobytes(), np.uint8)
+    head[18:26] = np.frombuffer(np.array([w, h], "<i4").tobytes(), np.uint8)
+    head[26:30] = np.frombuffer(np.array([1, 24], "<u2").tobytes(), np.uint8)
+    head[34:38] = np.frombuffer(np.uint32(body.size).tobytes(), np.uint8)
+    np.concatenate([head, body.reshape(-1)]).tofile(path)
+
+
+def stage_synth_data(dirpath, seed=1):
+    """Writes the layout CaffeEvaWrapper reads (AlexNet/Bin.Files/<ALEXNET_PFX>.*, AlexNet/imagenet_mean.single.bin,
+    Cls.Names/class_names.txt, Cls.Names/image_labels.txt) plus ten BMPs under Bmp.Files/, all from seeds: the AlexNet
+    of synth_alexnet(seed), a random mean image and random pictures of the sizes in SYNTH_BMP_SHAPES.  Returns the list
+    of BMP paths."""
+    rng = np.random.RandomState(seed + 1000)
+    save_model(os.path.join(dirpath, "AlexNet", "Bin.Files"), ALEXNET_PFX, synth_alexnet(seed))
+    write_bin(os.path.join(dirpath, "AlexNet", "imagenet_mean.single.bin"),
+              (rng.rand(3, 256, 256) * 120 + 60).astype(np.float32))
+    os.makedirs(os.path.join(dirpath, "Bmp.Files"), exist_ok=True)
+    os.makedirs(os.path.join(dirpath, "Cls.Names"), exist_ok=True)
+    paths = []
+    for i, (h, w) in enumerate(SYNTH_BMP_SHAPES, 1):
+        paths.append(os.path.join(dirpath, "Bmp.Files", "SYNTH_%08d.BMP" % i))
+        write_bmp(paths[-1], rng.randint(0, 256, size=(h, w, 3)).astype(np.uint8))
+    with open(os.path.join(dirpath, "Cls.Names", "class_names.txt"), "w") as f:
+        f.write("".join("class %d\n" % c for c in range(1000)))
+    with open(os.path.join(dirpath, "Cls.Names", "image_labels.txt"), "w") as f:
+        f.write("".join("SYNTH_%08d.JPEG %d\n" % (i, (37 * i) % 1000) for i in range(1, len(paths) + 1)))
+    return paths
+
+
+# ------------------------------------------------------------------------------------------------
 # whole-network oracle (the port): CaffeEva::ExecForwardPass(img, prob), src/CaffeEva.cc:213-261
 # ------------------------------------------------------------------------------------------------
 def net_forward(layers, params, img_nchw, keep=False):

@@ -11,7 +11,17 @@ Outputs (all small):
                     (inputs + parameters stored alongside)
   bmp_top5.npz      top-5 of CaffeEvaWrapper::Proc on the ten shipped BMPs + fingerprints of BmpImgIO::Load outputs
   cbn_vectors.npz   byte images of .cbn / .bin files written by the reference's own FileIO for 4/5/7/8-bit tables
+  synth_alexnet_kat.npz, synth_bmp_top5.npz
+                    the same as alexnet_kat.npz / bmp_top5.npz for the seeded data directory of
+                    pyoracle.stage_synth_data (synthetic AlexNet, mean image and BMPs): what the tests compare against
+                    where the reference's shipped files are not staged
+  live_ref.npz      reference GetInPdMat outputs and reference forward passes of seeded random conv / FC layers
+                    (fixed samples of the outputs + float64 checksums; inputs are regenerated from the seeds)
+  alexnet_live_ref.npz
+                    the reference's CaffeEva on LCG image 777, shipped and synthetic AlexNet: probabilities, samples +
+                    checksums of every feature map, SHA-256 of every decoded parameter buffer
 """
+import hashlib
 import os
 import sys
 import tempfile
@@ -20,13 +30,15 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from oracle import pyoracle as po  # noqa: E402
+from test_oracle_vs_reference import LUT_CASES, RANDOM_LAYER_CASES  # noqa: E402
 
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 
-def alexnet_kat():
-    net = po.RefNet(po.ALEXNET_DIR, po.ALEXNET_PFX)
+def alexnet_kat(dirpath=po.ALEXNET_DIR, name="alexnet_kat.npz"):
+    net = po.RefNet(dirpath, po.ALEXNET_PFX)
     imgs = po.lcg_images(2, 12345)
     out = {}
     for i in range(2):
@@ -45,7 +57,7 @@ def alexnet_kat():
         for l in (1, 5, 9, 11, 13, 16, 19, 22):
             out["fm%d_%d" % (l, i)] = net.featmap(l).reshape(-1)[:64].copy()
     net.close()
-    np.savez_compressed(os.path.join(OUT, "alexnet_kat.npz"), **out)
+    np.savez_compressed(os.path.join(OUT, name), **out)
 
 
 def synth_layers():
@@ -113,18 +125,20 @@ def cbn_vectors():
     np.savez_compressed(os.path.join(OUT, "cbn_vectors.npz"), **out)
 
 
-def bmp_top5():
+def bmp_top5(d=po.REF_DATA, bmps=None, name="bmp_top5.npz"):
     """CaffeEvaWrapper::Proc (reference src/CaffeEvaWrapper.cc:153-209) on the ten shipped BMPs + a fingerprint of
     BmpImgIO::Load's output tensor for each."""
     import ctypes as C
     R = po.ref()
     R.ref_wrapper_create.restype = C.c_void_p
-    d = po.REF_DATA
+    if bmps is None:
+        bmps = ["%s/Bmp.Files/ILSVRC2012_val_%08d.BMP" % (d, i) for i in range(1, 11)]
     h = C.c_void_p(R.ref_wrapper_create(d.encode(), (d + "/Cls.Names/class_names.txt").encode(),
                                         (d + "/Cls.Names/image_labels.txt").encode()))
+    assert h.value
     out = {}
-    for i in range(1, 11):
-        bmp = ("%s/Bmp.Files/ILSVRC2012_val_%08d.BMP" % (d, i)).encode()
+    for i, path in enumerate(bmps, 1):
+        bmp = path.encode()
         idx = np.zeros(5, np.int32)
         pr = np.zeros(5, np.float32)
         assert R.ref_wrapper_proc(h, bmp, 5, idx.ctypes.data_as(C.c_void_p), pr.ctypes.data_as(C.c_void_p)) == 0
@@ -135,7 +149,67 @@ def bmp_top5():
         out["top5_prob_%02d" % i] = pr
         out["img_cks_%02d" % i] = np.array([a.sum(), np.sqrt((a * a).sum()), a.max(), a.min()])
         out["img_head_%02d" % i] = img[:64].copy()
-    np.savez_compressed(os.path.join(OUT, "bmp_top5.npz"), **out)
+    np.savez_compressed(os.path.join(OUT, name), **out)
+
+
+def synth_data():
+    """alexnet_kat / bmp_top5 on the seeded stand-in of the reference's data directory."""
+    with tempfile.TemporaryDirectory() as tmp:
+        bmps = po.stage_synth_data(tmp)
+        alexnet_kat(os.path.join(tmp, "AlexNet", "Bin.Files"), "synth_alexnet_kat.npz")
+        bmp_top5(tmp, bmps, "synth_bmp_top5.npz")
+
+
+def alexnet_live_ref():
+    out = {}
+    with tempfile.TemporaryDirectory() as tmp:
+        po.stage_synth_data(tmp)
+        for key, dirpath in (("shipped", po.ALEXNET_DIR), ("synth", os.path.join(tmp, "AlexNet", "Bin.Files"))):
+            net = po.RefNet(dirpath, po.ALEXNET_PFX)
+            out[key + "_prob"] = net.forward(po.lcg_images(1, 777)[0])
+            for l in range(24):
+                out["%s_fm%d_idx" % (key, l)], out["%s_fm%d_val" % (key, l)], out["%s_fm%d_cks" % (key, l)] = \
+                    sample(net.featmap(l), 64)
+            for l in po.ALEXNET_PQ:
+                for which, name in ((0, "bias"), (1, "ctrd"), (2, "asmt")):
+                    a, _ = net.param(l, which)
+                    out["%s_%s%d_sha256" % (key, name, l)] = np.array(hashlib.sha256(a.tobytes()).hexdigest())
+            net.close()
+    np.savez_compressed(os.path.join(OUT, "alexnet_live_ref.npz"), **out)
+
+
+def sample(a, n=512):
+    """A fixed sample of a flattened output (indices, values) and its float64 (sum, l2, max)."""
+    a = np.ascontiguousarray(a, np.float32).reshape(-1)
+    idx = np.sort(np.random.RandomState(a.size).choice(a.size, min(n, a.size), replace=False))
+    m = a.astype(np.float64)
+    return idx, a[idx], np.array([m.sum(), np.sqrt((m * m).sum()), m.max()])
+
+
+def live_ref():
+    """Inputs of tests/test_oracle_vs_reference.py's LUT-stage and random-layer tests (same seeds, same order), through
+    the reference."""
+    out = {}
+    rng = np.random.RandomState(11)
+    for c, (P, D, S, K, d) in enumerate(LUT_CASES):
+        data = (rng.randn(P, D) * 10).astype(np.float32)
+        ctrd = (rng.randn(S, K, d) * 0.1).astype(np.float32)
+        out["lut%d_idx" % c], out["lut%d_val" % c], out["lut%d_cks" % c] = sample(po.ref_get_inpd(data, ctrd))
+    rng = np.random.RandomState(99)
+    with tempfile.TemporaryDirectory() as tmp:
+        for ci, (layers, chw, pq) in enumerate(RANDOM_LAYER_CASES):
+            params = po.synth_model(layers, chw, pq, seed=ci, ctrd_std=0.2)
+            d = os.path.join(tmp, "m%d" % ci)
+            po.save_model(d, "rnd", params)
+            net = po.RefNet(d, "rnd", layers=layers, in_chw=chw)
+            a, _ = net.param(0, 2)
+            out["rnd%d_asmt_sha256" % ci] = np.array(hashlib.sha256(a.tobytes()).hexdigest())
+            for j in range(2):
+                img = (rng.randn(*chw) * 5).astype(np.float32)
+                out["rnd%d_%d_idx" % (ci, j)], out["rnd%d_%d_val" % (ci, j)], out["rnd%d_%d_cks" % (ci, j)] = \
+                    sample(net.forward(img))
+            net.close()
+    np.savez_compressed(os.path.join(OUT, "live_ref.npz"), **out)
 
 
 if __name__ == "__main__":
@@ -145,5 +219,8 @@ if __name__ == "__main__":
     synth_layers()
     cbn_vectors()
     bmp_top5()
+    synth_data()
+    live_ref()
+    alexnet_live_ref()
     for f in sorted(os.listdir(OUT)):
         print(f, os.path.getsize(os.path.join(OUT, f)))

@@ -2,7 +2,8 @@
 (qcnn_preproc_*), the uint8 entry points of the network, and the k-fold arg-max (qcnn_topk).
 
 Bars: preprocessing BIT-IDENTICAL to the CPU path (the C++ host port, itself pinned bit-for-bit to the compiled reference
-by tests/test_host_mirror.py, and the reference fingerprints in tests/golden/bmp_top5.npz); top-k identical to the
+by tests/test_host_mirror.py, and the reference fingerprints in tests/golden/bmp_top5.npz, or synth_bmp_top5.npz for
+the seeded stand-in of the ref_data fixture); top-k identical to the
 oracle's restatement of CaffeEvaWrapper::Proc, ties included; uint8 entry == fp32 entry on (float)pixel - mean, bit for bit."""
 import ctypes as C
 import os
@@ -12,10 +13,6 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG = os.path.join(ROOT, "quantized-cnn_b200")
-DATA = os.path.join(ROOT, "oracle", "_ref", "data")
-GOLD = os.path.join(ROOT, "tests", "golden")
-needs_data = pytest.mark.skipif(not os.path.exists(os.path.join(DATA, "Bmp.Files", "ILSVRC2012_val_00000010.BMP")),
-                                reason="reference fixtures not staged under oracle/_ref/data")
 
 
 def decode_bmp(path):
@@ -72,15 +69,14 @@ def resz_crop_numpy(img, mean, full, crop, relaxed, mean_full):
 
 
 @pytest.mark.gpu
-@needs_data
-def test_device_bmp_preprocessing_is_bit_identical_to_the_cpu_path(po, qcnn, ctx):
+def test_device_bmp_preprocessing_is_bit_identical_to_the_cpu_path(po, qcnn, ctx, ref_data):
     host = C.CDLL(os.path.join(PKG, "libqcnn_host.so"))
-    g = np.load(os.path.join(GOLD, "bmp_top5.npz"))
-    mean_path = os.path.join(DATA, "AlexNet", "imagenet_mean.single.bin")
+    g = ref_data["bmp"]
+    mean_path = ref_data["mean"]
     mean = po.read_bin(mean_path)
     assert mean.shape == (3, 256, 256)
     pp = qcnn.Preproc(ctx, mean)           # AlexNet recipe of CaffeEvaWrapper::SetModel: Strict 256x256, full mean, crop 227
-    paths = [os.path.join(DATA, "Bmp.Files", "ILSVRC2012_val_%08d.BMP" % i) for i in range(1, 11)]
+    paths = ref_data["bmps"]
     imgs = [decode_bmp(p) for p in paths]
     assert len({im.shape for im in imgs}) > 1          # pictures of different sizes in ONE launch
     got = pp.run(imgs).cpu().numpy()

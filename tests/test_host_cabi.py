@@ -78,13 +78,12 @@ def test_cbn_edge_cases_against_oracle(qcnn, po, tmp_path):
             assert np.array_equal(got2, idx0)
 
 
-def test_shipped_alexnet_files_decode_identically(qcnn, po):
-    if not po.have_alexnet():
-        pytest.skip("shipped AlexNet parameters not staged")
+def test_shipped_alexnet_files_decode_identically(qcnn, po, ref_data):
+    """The AlexNet parameter files of the ref_data fixture: the reference's shipped ones where they are staged."""
     layers = po.alexnet_layers()
-    params = po.load_model(po.ALEXNET_DIR, po.ALEXNET_PFX, layers)
+    params = po.load_model(ref_data["model_dir"], po.ALEXNET_PFX, layers)
     for l, p in params.items():
-        base = os.path.join(po.ALEXNET_DIR, po.ALEXNET_PFX)
+        base = os.path.join(ref_data["model_dir"], po.ALEXNET_PFX)
         a, bits = qcnn.read_cbn_u8("%s.asmtLst.%02d.cbn" % (base, l + 1))
         assert bits == p["bits"] and np.array_equal(a, p["asmt"])
         S, K, d = p["ctrd"].shape

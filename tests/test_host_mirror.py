@@ -1,6 +1,7 @@
 """The C++ host layer that keeps the reference's class API (CaffeEvaWrapper / CaffeEva / CaffePara / BmpImgIO):
 CPU-side pieces are checked here against golden data produced by the compiled reference; the GPU-side end-to-end
-classification of the reference's ten BMP fixtures is gpu-marked."""
+classification of ten BMP fixtures is gpu-marked.  The data directory is the ref_data fixture's: the reference's
+shipped model, mean image and BMPs where they are staged, else a seeded stand-in with the reference's outputs on it."""
 import ctypes as C
 import os
 import subprocess
@@ -10,12 +11,7 @@ import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-GOLD = os.path.join(HERE, "golden")
 PKG = os.path.join(ROOT, "quantized-cnn_b200")
-DATA = os.path.join(ROOT, "oracle", "_ref", "data")
-
-needs_data = pytest.mark.skipif(not os.path.exists(os.path.join(DATA, "Bmp.Files")),
-                                reason="reference fixtures not staged (oracle/_ref/data)")
 
 
 def hostlib():
@@ -41,13 +37,12 @@ def test_layer_tables_match_reference_counts():
     assert lib.qcnn_host_layer_table(b"ResNet", chw, types, 64) == -1
 
 
-@needs_data
-def test_bmp_preprocessing_matches_reference_bit_for_bit():
+def test_bmp_preprocessing_matches_reference_bit_for_bit(ref_data):
     lib = hostlib()
-    g = np.load(os.path.join(GOLD, "bmp_top5.npz"))
-    mean = os.path.join(DATA, "AlexNet", "imagenet_mean.single.bin").encode()
-    for i in range(1, 11):
-        bmp = os.path.join(DATA, "Bmp.Files", "ILSVRC2012_val_%08d.BMP" % i).encode()
+    g = ref_data["bmp"]
+    mean = ref_data["mean"].encode()
+    for i, path in enumerate(ref_data["bmps"], 1):
+        bmp = path.encode()
         out = np.zeros(3 * 227 * 227, np.float32)
         n = lib.qcnn_host_load_bmp_alexnet(mean, bmp, out.ctypes.data_as(C.c_void_p), out.size)
         assert n == out.size
@@ -58,15 +53,16 @@ def test_bmp_preprocessing_matches_reference_bit_for_bit():
 
 
 @pytest.mark.gpu
-@needs_data
 @pytest.mark.parametrize("mode", ["strict", "default"])
-def test_wrapper_classifies_reference_bmps_like_the_reference(mode):
+def test_wrapper_classifies_reference_bmps_like_the_reference(mode, ref_data):
     """quancnn_b200 classify == UnitTest::UT_CaffeEvaWrapper (reference src/UnitTest.cc:67-124) on the ten fixtures;
-    expected top-5 from the compiled reference (tests/golden/bmp_top5.npz == SURVEY.md Appendix B)."""
-    g = np.load(os.path.join(GOLD, "bmp_top5.npz"))
-    bmps = [os.path.join(DATA, "Bmp.Files", "ILSVRC2012_val_%08d.BMP" % i) for i in range(1, 11)]
-    cmd = [os.path.join(PKG, "quancnn_b200"), "classify", DATA, os.path.join(DATA, "Cls.Names", "class_names.txt"),
-           os.path.join(DATA, "Cls.Names", "image_labels.txt"), "5"] + bmps
+    expected top-5 from the compiled reference (tests/golden/bmp_top5.npz == SURVEY.md Appendix B for the shipped
+    fixtures, tests/golden/synth_bmp_top5.npz for the stand-in)."""
+    g = ref_data["bmp"]
+    data = ref_data["dir"]
+    bmps = ref_data["bmps"]
+    cmd = [os.path.join(PKG, "quancnn_b200"), "classify", data, os.path.join(data, "Cls.Names", "class_names.txt"),
+           os.path.join(data, "Cls.Names", "image_labels.txt"), "5"] + bmps
     # strict: LUT + gather kernels only (QCNN_NO_DECTC / QCNN_FC_TC=0), probabilities within 2e-5 of the reference;
     # default: decode-at-use tensor-core kernels allowed, within 2e-4 (tolerances: tests/test_gpu_net.py)
     env = dict(os.environ)
@@ -95,26 +91,27 @@ def test_wrapper_classifies_reference_bmps_like_the_reference(mode):
 
 
 @pytest.mark.gpu
-@needs_data
-def test_per_layer_members_agree_with_fused_network():
+def test_per_layer_members_agree_with_fused_network(ref_data):
     """CaffeEva::CalcFeatMap_* driven layer by layer with host matrices (the reference executor's calling pattern)
     reproduces the fused device-resident forward pass."""
-    out = subprocess.run([os.path.join(PKG, "quancnn_b200"), "layers", DATA], capture_output=True, text=True, timeout=600)
+    out = subprocess.run([os.path.join(PKG, "quancnn_b200"), "layers", ref_data["dir"]], capture_output=True, text=True,
+                         timeout=600)
     assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
     line = [l for l in out.stdout.splitlines() if l.startswith("LAYERS")][0]
-    assert "argmax0=533" in line            # SURVEY.md Appendix B synthetic KAT
+    # the reference's class for LCG image 12345 (533 with the shipped model: SURVEY.md Appendix B synthetic KAT)
+    assert "argmax0=%d " % int(ref_data["kat"]["top5_0"][0]) in line
     # probabilities of the layer-by-layer run (host matrices between layers, un-fused kernels) vs the fused device pass
     err = float(line.split("max|layerwise-fused|=")[1])
     assert err <= 2e-5, line
 
 
 @pytest.mark.gpu
-@needs_data
-def test_host_executor_shards_over_all_gpus():
+def test_host_executor_shards_over_all_gpus(ref_data):
     """CaffeEva::SetDeviceCount(n): ExecForwardPass through qcnn_multi_* (n = every GPU of the box, 1 included)."""
     import torch
     n = max(1, min(torch.cuda.device_count(), 8))
-    out = subprocess.run([os.path.join(PKG, "quancnn_b200"), "layers", DATA, str(n)], capture_output=True, text=True, timeout=600)
+    out = subprocess.run([os.path.join(PKG, "quancnn_b200"), "layers", ref_data["dir"], str(n)], capture_output=True,
+                         text=True, timeout=600)
     assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
     line = [l for l in out.stdout.splitlines() if l.startswith("LAYERS")][0]
-    assert "argmax0=533" in line
+    assert "argmax0=%d " % int(ref_data["kat"]["top5_0"][0]) in line

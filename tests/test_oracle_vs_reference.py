@@ -1,12 +1,13 @@
-"""Pins the CPU oracle (oracle/pq_oracle.c): bit-for-bit against
-  (1) the committed golden vectors generated from the compiled reference (tests/golden/make_golden.py), always;
-  (2) the compiled reference itself (oracle/_ref/libqcnn_ref.so) when it is present (it is built from the
-      unmodified /root/reference sources by oracle/Makefile and travels git-ignored).
-No GPU, no product code."""
+"""Pins the CPU oracle (oracle/pq_oracle.c) bit-for-bit against golden vectors generated from the compiled reference
+(tests/golden/make_golden.py; the reference is built from its unmodified sources by oracle/Makefile, and the vectors
+travel with the repository).  No GPU, no product code."""
+import hashlib
 import os
 
 import numpy as np
 import pytest
+
+from oracle import pyoracle
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -96,13 +97,12 @@ def test_lcg_image_generator(po):
     assert img.min() >= -128 and img.max() < 128
 
 
-def test_oracle_alexnet_kat_matches_reference_golden(po):
-    """Shipped quantized AlexNet (staged under oracle/_ref/data by oracle/Makefile) through the oracle port."""
-    if not po.have_alexnet():
-        pytest.skip("shipped AlexNet parameters not staged (oracle/_ref/data)")
-    g = golden("alexnet_kat.npz")
+def test_oracle_alexnet_kat_matches_reference_golden(po, ref_data):
+    """AlexNet through the oracle port: the reference's shipped parameter files where they are staged under
+    oracle/_ref/data, else the seeded synthetic AlexNet of pyoracle.stage_synth_data."""
+    g = ref_data["kat"]
     layers = po.alexnet_layers()
-    params = po.load_model(po.ALEXNET_DIR, po.ALEXNET_PFX, layers)
+    params = po.load_model(ref_data["model_dir"], po.ALEXNET_PFX, layers)
     imgs = po.lcg_images(2, 12345)
     for i in range(2):
         prob, maps = po.net_forward(layers, params, imgs[i:i + 1], keep=True)
@@ -116,68 +116,70 @@ def test_oracle_alexnet_kat_matches_reference_golden(po):
         for l in range(24):
             m = maps[l].astype(np.float64).reshape(-1)
             assert np.allclose([m.sum(), np.sqrt((m * m).sum()), m.max()], cks[l], rtol=1e-12, atol=0)
-    # SURVEY.md Appendix B: seed 12345 -> class 533, p = 0.621259
-    assert int(g["top5_0"][0]) == 533 and abs(float(g["prob0"][533]) - 0.621259) < 1e-6
+    if ref_data["shipped"]:
+        # SURVEY.md Appendix B: seed 12345 -> class 533, p = 0.621259
+        assert int(g["top5_0"][0]) == 533 and abs(float(g["prob0"][533]) - 0.621259) < 1e-6
 
 
-# ---- live cross-checks against the compiled reference (present in the build container and on the GPU box) ----
-needs_ref = pytest.mark.skipif(not os.path.exists(os.path.join(os.path.dirname(GOLD), "..", "oracle", "_ref",
-                                                               "libqcnn_ref.so")), reason="oracle/_ref not built")
+# ---- seeded cases whose reference outputs are stored in tests/golden/live_ref.npz (make_golden.py: live_ref) ----
+LUT_CASES = [(50, 48, 6, 128, 8), (7, 3, 1, 128, 8), (3, 10, 3, 32, 4), (2, 4096, 4096, 16, 1)]
+RANDOM_LAYER_CASES = [
+    ([pyoracle.conv(1, 3, 64, 2, 1)], (32, 13, 13), {0: (4, 64, 4)}),
+    ([pyoracle.conv(2, 5, 48, 1, 2)], (6, 17, 15), {0: (2, 128, 4)}),      # d > remaining dims in last subspace
+    ([pyoracle.conv(0, 11, 32, 1, 4)], (3, 51, 51), {0: (1, 128, 8)}),
+    ([pyoracle.fcnt(64)], (30, 2, 2), {0: (30, 32, 4)}),
+    ([pyoracle.fcnt(1000)], (100, 1, 1), {0: (100, 16, 1)}),
+]
 
 
-@needs_ref
+def assert_matches_sample(out, g, key):
+    """out bit-identical to the reference at the stored sample positions, and its float64 (sum, l2, max) equal."""
+    out = out.reshape(-1)
+    assert np.array_equal(out[g[key + "_idx"]], g[key + "_val"]), key
+    m = out.astype(np.float64)
+    assert np.allclose([m.sum(), np.sqrt((m * m).sum()), m.max()], g[key + "_cks"], rtol=1e-12, atol=0), key
+
+
 def test_oracle_lut_stage_matches_live_reference(po):
+    g = golden("live_ref.npz")
     rng = np.random.RandomState(11)
-    for (P, D, S, K, d) in [(50, 48, 6, 128, 8), (7, 3, 1, 128, 8), (3, 10, 3, 32, 4), (2, 4096, 4096, 16, 1)]:
+    for c, (P, D, S, K, d) in enumerate(LUT_CASES):
         data = (rng.randn(P, D) * 10).astype(np.float32)
         ctrd = (rng.randn(S, K, d) * 0.1).astype(np.float32)
-        assert np.array_equal(po.get_inpd(data, ctrd), po.ref_get_inpd(data, ctrd))
+        assert_matches_sample(po.get_inpd(data, ctrd), g, "lut%d" % c)
 
 
-@needs_ref
 def test_oracle_random_layers_match_live_reference(po, tmp_path):
-    """Seeded random conv / FC shapes through the reference's own CalcFeatMap_ConvAprx / _FCntAprx."""
+    """Seeded random conv / FC shapes against the reference's own CalcFeatMap_ConvAprx / _FCntAprx."""
+    g = golden("live_ref.npz")
     rng = np.random.RandomState(99)
-    cases = [
-        ([po.conv(1, 3, 64, 2, 1)], (32, 13, 13), {0: (4, 64, 4)}),
-        ([po.conv(2, 5, 48, 1, 2)], (6, 17, 15), {0: (2, 128, 4)}),      # d > remaining dims in last subspace
-        ([po.conv(0, 11, 32, 1, 4)], (3, 51, 51), {0: (1, 128, 8)}),
-        ([po.fcnt(64)], (30, 2, 2), {0: (30, 32, 4)}),
-        ([po.fcnt(1000)], (100, 1, 1), {0: (100, 16, 1)}),
-    ]
-    for ci, (layers, chw, pq) in enumerate(cases):
+    for ci, (layers, chw, pq) in enumerate(RANDOM_LAYER_CASES):
         params = po.synth_model(layers, chw, pq, seed=ci, ctrd_std=0.2)
         d = str(tmp_path / ("m%d" % ci))
         po.save_model(d, "rnd", params)
-        net = po.RefNet(d, "rnd", layers=layers, in_chw=chw)
-        # decoded parameters identical (bit-exact assignment indexing)
-        a, _ = net.param(0, 2)
-        assert np.array_equal(a, params[0]["asmt"].reshape(-1))
-        for _ in range(2):
+        # decoded parameters identical (bit-exact assignment indexing): the oracle reads back what the reference read
+        a, _ = po.read_cbn(os.path.join(d, "rnd.asmtLst.01.cbn"))
+        assert np.array_equal(a, params[0]["asmt"])
+        assert hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest() == str(g["rnd%d_asmt_sha256" % ci])
+        for j in range(2):
             img = (rng.randn(*chw) * 5).astype(np.float32)
-            ref = net.forward(img)
-            mine = po.net_forward(layers, params, img[None])
-            assert np.array_equal(mine.reshape(-1), ref)
-        net.close()
+            assert_matches_sample(po.net_forward(layers, params, img[None]), g, "rnd%d_%d" % (ci, j))
 
 
-@needs_ref
-def test_alexnet_live_reference_vs_oracle(po):
-    if not po.have_alexnet():
-        pytest.skip("shipped AlexNet parameters not staged")
-    net = po.RefNet(po.ALEXNET_DIR, po.ALEXNET_PFX)
+def test_alexnet_live_reference_vs_oracle(po, ref_data):
+    """The reference's CaffeEva on LCG image 777 (tests/golden/alexnet_live_ref.npz, for the shipped and the synthetic
+    AlexNet of the ref_data fixture): probabilities, every feature map and every decoded parameter buffer."""
+    g = golden("alexnet_live_ref.npz")
+    key = "shipped" if ref_data["shipped"] else "synth"
     layers = po.alexnet_layers()
-    params = po.load_model(po.ALEXNET_DIR, po.ALEXNET_PFX, layers)
-    img = po.lcg_images(1, 777)
-    ref = net.forward(img[0])
-    mine, maps = po.net_forward(layers, params, img, keep=True)
-    assert np.array_equal(mine[0], ref)
+    params = po.load_model(ref_data["model_dir"], po.ALEXNET_PFX, layers)
+    mine, maps = po.net_forward(layers, params, po.lcg_images(1, 777), keep=True)
+    assert np.array_equal(mine[0], g[key + "_prob"])
     for l in range(24):
         if l == 15:
             continue  # reference leaves featMapLst[15] in NCHW order (CaffeEva.cc:246-253)
-        assert np.array_equal(maps[l].reshape(-1), net.featmap(l).reshape(-1)), l
+        assert_matches_sample(maps[l], g, "%s_fm%d" % (key, l))
     for l in params:
-        for which, key in ((0, "bias"), (1, "ctrd"), (2, "asmt")):
-            a, _ = net.param(l, which)
-            assert np.array_equal(a, params[l][key].reshape(-1))
-    net.close()
+        for name in ("bias", "ctrd", "asmt"):
+            a = np.ascontiguousarray(params[l][name])
+            assert hashlib.sha256(a.tobytes()).hexdigest() == str(g["%s_%s%d_sha256" % (key, name, l)]), (l, name)
